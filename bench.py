@@ -19,6 +19,9 @@ meet in the timing barrier.
   roofline: dominant kernel (by summed device time inside the forward, CUDA events on the compute stream)
            against the measured tensor peak in MEASURED_PEAKS.json.
   cpu_baseline: the oracle's HF-transformers fp32 path on the host cores (N=1, rank 0, bounded sample).
+
+--dump-outputs DIR writes the embeddings the timed path returned in its last step to DIR/embeddings.npy (see dump_outputs);
+weights and inputs are seeded, so two builds run with the same arguments can be compared row for row.
 """
 import argparse
 import json
@@ -30,6 +33,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True  # the tree may be read-only: the benchmark writes nothing into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "modal-examples_b200"))
 
@@ -48,6 +52,20 @@ KERNEL_FLOPS = {
 # algorithmic HBM bytes per token of the row-wise kernels (DESIGN.md §4): embedding gather = one fp32 word row in, the
 # residual stream out as fp16 hi + fp16 lo, six (sum, M2) partials.  (There is no LayerNorm kernel any more.)
 KERNEL_BYTES = {"embed": 3072 + 1536 + 1536 + 48}
+DUMP_BYTES = 64 << 20          # --dump-outputs writes at most this much
+
+
+def dump_outputs(path, emb):
+    """Writes `emb` (one embedding per item, in input order) as PATH/embeddings.npy in float32.  Beyond DUMP_BYTES a fixed
+    sample of rows (numpy default_rng(0), kept in input order) stands in for the whole, the same rows on every run."""
+    import numpy as np
+
+    emb = np.asarray(emb, dtype=np.float32)
+    keep = (DUMP_BYTES - 4096) // (emb.shape[1] * 4)  # 4096: room for the .npy header
+    if len(emb) > keep:
+        emb = emb[np.sort(np.random.default_rng(0).choice(len(emb), keep, replace=False))]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "embeddings.npy"), emb)
 
 
 def load_peaks():
@@ -190,6 +208,8 @@ def main_reference(args):
         "cpu_baseline": {"value": value, "unit": "items/s", "cores": threads, "host_cores": os.cpu_count(), "kind": "port", "sample": sample},
         "e2e": {"value": value, "unit": "items/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     GUARD.emit(json.dumps(line))
     return 0
 
@@ -611,6 +631,8 @@ def main_ours(args):
         line["independent_replicas"] = indep
     if cpu_baseline:
         line["cpu_baseline"] = cpu_baseline
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dev_out)  # the headline device-resident loop's last step, every replica in item order
     GUARD.emit(json.dumps(line))
     pin_ids.free()
     pin_out.free()
@@ -649,7 +671,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-vit", action="store_true", help="skip the secondary CLIP ViT-B/16 measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's embeddings to DIR/embeddings.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3  # timing rule: W >= 3
     sys.exit(main_reference(args) if args.impl == "reference" else main_ours(args))

@@ -6,6 +6,7 @@ import re
 import subprocess
 
 import pytest
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -43,7 +44,7 @@ def test_library_is_blackwell_native():
     assert "HMMA.16816" not in sass, "legacy mma.sync path found"
 
 
-@pytest.mark.skipif(os.path.exists("/dev/nvidia0"), reason="GPU present")
+@pytest.mark.skipif(torch.cuda.is_available(), reason="GPU present")
 def test_no_cpu_fallback():
     """Product path must fail loudly without a GPU."""
     import b200rt

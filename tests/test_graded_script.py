@@ -1,5 +1,5 @@
 """CPU: the graded reference script runs VERBATIM through the `modal` shim --
-`modal run /root/reference/06_gpu_and_ml/embeddings/text_embeddings_inference.py::embed_dataset` (:141-169): the volume at
+`modal run 06_gpu_and_ml/embeddings/text_embeddings_inference.py::embed_dataset` (:141-169): the volume at
 /data (virtual mount, nothing created under /), `spawn_server()` Popen + TCP readiness (:37-51), the `@app.cls` /
 `@modal.concurrent` / `@modal.enter` / async `@modal.method` class (:79-104), `generate_batches()` (batches of 32, remainder
 dropped, :156-163) and `model.embed.map(..., order_outputs=False)` (:167).  The `text-embeddings-router` on PATH is the
@@ -13,10 +13,10 @@ import sys
 
 import pytest
 
+from oracle.stage_modal_examples import staged
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "modal-examples_b200")
-REF = "/root/reference"
-SCRIPT = os.path.join(REF, "06_gpu_and_ml", "embeddings", "text_embeddings_inference.py")
 
 
 def _port_free(port):
@@ -28,9 +28,9 @@ def _port_free(port):
             return False
 
 
-@pytest.mark.skipif(not os.path.exists(SCRIPT), reason="reference tree not present on this box")
 @pytest.mark.timeout(600)
 def test_text_embeddings_inference_embed_dataset_runs_unchanged(tmp_path):
+    script = staged("06_gpu_and_ml/embeddings/text_embeddings_inference.py")
     if not _port_free(8000):
         pytest.skip("port 8000 (hard-coded in the reference script) is taken on this box")
     state = tmp_path / "state"
@@ -42,7 +42,7 @@ def test_text_embeddings_inference_embed_dataset_runs_unchanged(tmp_path):
     assert r.returncode == 0, r.stderr
     data = json.load(open(state / "volumes" / "tei-hn-data" / "dataset.jsonl"))
     assert len(data) == rows and not os.path.exists("/data/dataset.jsonl")
-    r = subprocess.run([sys.executable, "-m", "modal", "run", SCRIPT + "::embed_dataset"], env=env, capture_output=True, text=True, timeout=540)
+    r = subprocess.run([sys.executable, "-m", "modal", "run", script + "::embed_dataset"], env=env, capture_output=True, text=True, timeout=540)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-4000:])
     assert "Webserver ready!" in r.stdout
     reqs = [json.loads(l) for l in open(tmp_path / "tei.jsonl")]

@@ -10,8 +10,8 @@ import time
 import pytest
 
 import modal
+from oracle.stage_modal_examples import staged
 
-REF = "/root/reference"
 PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "modal-examples_b200")
 
 
@@ -307,7 +307,6 @@ def test_cli_runs_entrypoint_with_kebab_options(tmp_path):
     assert r.returncode == 0 and r.stdout.strip().endswith("49")
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this box")
 @pytest.mark.parametrize("rel,expect", [
     ("01_getting_started/hello_world.py", "2646700"),
     ("01_getting_started/generators.py", "9"),
@@ -315,20 +314,18 @@ def test_cli_runs_entrypoint_with_kebab_options(tmp_path):
     ("03_scaling_out/dynamic_batching.py", "ASCII codes: [33, 34, 35, 36, 37, 38]"),
 ])
 def test_reference_scripts_run_unchanged(rel, expect):
-    r = _cli("run", os.path.join(REF, rel))
+    r = _cli("run", staged(rel))
     assert r.returncode == 0, r.stderr[-2000:]
     assert expect in r.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not present on this box")
 def test_reference_hot_path_scripts_import_unchanged():
     """The reference's own smoke test is `importlib.import_module` of every example
     (internal/examples_test.py:39-41); here over the embeddings directory with the shim as `modal`."""
     import importlib.util
 
-    base = os.path.join(REF, "06_gpu_and_ml", "embeddings")
     for fn in ["text_embeddings_inference.py", "amazon_embeddings.py", "image_embeddings_infinity.py", "qdrant.py"]:
-        spec = importlib.util.spec_from_file_location("refmod_" + fn[:-3], os.path.join(base, fn))
+        spec = importlib.util.spec_from_file_location("refmod_" + fn[:-3], staged("06_gpu_and_ml/embeddings/" + fn))
         mod = importlib.util.module_from_spec(spec)
         spec.loader.exec_module(mod)
         assert any(isinstance(v, modal.App) for v in vars(mod).values())

@@ -28,13 +28,11 @@ import sys
 import numpy as np
 import pytest
 
+from oracle.stage_modal_examples import staged
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "modal-examples_b200")
-EMB = "/root/reference/06_gpu_and_ml/embeddings"
-WIKI = os.path.join(EMB, "wikipedia", "main.py")
-AMAZON = os.path.join(EMB, "amazon_embeddings.py")
-INFINITY = os.path.join(EMB, "image_embeddings_infinity.py")
-SNAPSHOT = "/root/reference/06_gpu_and_ml/gpu_snapshot.py"
+EMB = "06_gpu_and_ml/embeddings/"
 
 
 def _port_free(port):
@@ -65,9 +63,9 @@ def _articles(n, seed):
     return out
 
 
-@pytest.mark.skipif(not os.path.exists(WIKI), reason="reference tree not present on this box")
 @pytest.mark.timeout(600)
 def test_wikipedia_embed_dataset_runs_unchanged(tmp_path):
+    wiki = staged(EMB + "wikipedia/main.py")
     if not _port_free(8000):
         pytest.skip("port 8000 (hard-coded in the reference script) is taken on this box")
     state, env = _env(tmp_path)
@@ -77,7 +75,7 @@ def test_wikipedia_embed_dataset_runs_unchanged(tmp_path):
     json.dump(arts, open(ds_dir / "train.json", "w"))
     chunks = [(a["id"], a["url"], a["title"], a["text"][s:s + 512]) for a in arts for s in range(0, len(a["text"]), 512)]
     batch_size = 4  # map inputs of 4 chunks (the script's default is 512 * 50)
-    r = subprocess.run([sys.executable, "-m", "modal", "run", WIKI + "::embed_dataset", "--down-scale", "1", "--batch-size", str(batch_size)],
+    r = subprocess.run([sys.executable, "-m", "modal", "run", wiki + "::embed_dataset", "--down-scale", "1", "--batch-size", str(batch_size)],
                        env=env, capture_output=True, text=True, timeout=540)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-4000:])
     assert "Webserver ready!" in r.stdout and "Saved checkpoint at /checkpoint/bge-small-en-v1.5-4" in r.stdout
@@ -103,9 +101,9 @@ def test_wikipedia_embed_dataset_runs_unchanged(tmp_path):
     assert hf[1]["folder_path"] == "/checkpoint/bge-small-en-v1.5-4" and "data.parquet" in hf[1]["files"]
 
 
-@pytest.mark.skipif(not os.path.exists(AMAZON), reason="reference tree not present on this box")
 @pytest.mark.timeout(600)
 def test_amazon_embeddings_entrypoint_runs_unchanged(tmp_path):
+    amazon = staged(EMB + "amazon_embeddings.py")
     if not _port_free(8000):
         pytest.skip("port 8000 (the reference script's default) is taken on this box")
     state, env = _env(tmp_path)
@@ -122,7 +120,7 @@ def test_amazon_embeddings_entrypoint_runs_unchanged(tmp_path):
     out_path = "/tmp/embeddings-example-fc-ids.json"  # written by the script's entrypoint (:55-61)
     if os.path.exists(out_path):
         os.remove(out_path)
-    r = subprocess.run([sys.executable, "-m", "modal", "run", "--detach", AMAZON, "--dataset-subset", "raw_review_Magazine_Subscriptions",
+    r = subprocess.run([sys.executable, "-m", "modal", "run", "--detach", amazon, "--dataset-subset", "raw_review_Magazine_Subscriptions",
                         "--down-scale", "1"], env=env, capture_output=True, text=True, timeout=540)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-4000:])
     assert "Inference server ready!" in r.stdout and "output handles saved to" in r.stdout
@@ -137,9 +135,9 @@ def test_amazon_embeddings_entrypoint_runs_unchanged(tmp_path):
     assert sorted(t for q in reqs for t in q["inputs"]) == sorted(c[-1] for c in chunks)
 
 
-@pytest.mark.skipif(not os.path.exists(INFINITY), reason="reference tree not present on this box")
 @pytest.mark.timeout(600)
 def test_image_embeddings_infinity_entrypoint_runs_unchanged(tmp_path):
+    infinity = staged(EMB + "image_embeddings_infinity.py")
     pytest.importorskip("torchvision")
     from PIL import Image
 
@@ -153,7 +151,7 @@ def test_image_embeddings_infinity_entrypoint_runs_unchanged(tmp_path):
     n = 7
     for i in range(n):
         Image.fromarray(rng.integers(0, 256, (224, 224, 3), dtype=np.uint8)).save(img_dir / f"img{i:07d}.jpg", quality=95)
-    r = subprocess.run([sys.executable, "-m", "modal", "run", INFINITY], env=env, capture_output=True, text=True, timeout=540)
+    r = subprocess.run([sys.executable, "-m", "modal", "run", infinity], env=env, capture_output=True, text=True, timeout=540)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-4000:])
     assert f"Found {n} JPEGs in the Volume." in r.stdout and "Loading 4 models..." in r.stdout
     assert f"n_ims={n}::concurrency=4" in r.stdout and "Embedding-only throughput (avg)" in r.stdout
@@ -162,20 +160,20 @@ def test_image_embeddings_infinity_entrypoint_runs_unchanged(tmp_path):
     assert [c["n"] for c in calls] == [n] and all(sz == [224, 224] for sz in calls[0]["sizes"])  # one map input of <= 100 images
 
 
-@pytest.mark.skipif(not os.path.exists(SNAPSHOT), reason="reference tree not present on this box")
 @pytest.mark.timeout(600)
 def test_gpu_snapshot_deploy_then_client_process(tmp_path):
+    snapshot = staged("06_gpu_and_ml/gpu_snapshot.py")
     state, env = _env(tmp_path, stubs=("stubs_st",))
     env["FAKE_ST_LAYERS"] = "1"
     # a client before any deployment: the script's own NotFoundError branch (:73-77)
-    r = subprocess.run([sys.executable, SNAPSHOT], env=env, capture_output=True, text=True, timeout=300)
+    r = subprocess.run([sys.executable, snapshot], env=env, capture_output=True, text=True, timeout=300)
     # (the app object exists in the client process because the client IS the app's file; it must still run)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-3000:])
-    r = subprocess.run([sys.executable, "-m", "modal", "deploy", SNAPSHOT], env=env, capture_output=True, text=True, timeout=300)
+    r = subprocess.run([sys.executable, "-m", "modal", "deploy", snapshot], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "deployed app 'example-gpu-snapshot'" in r.stdout, (r.stdout[-2000:], r.stderr[-3000:])
     reg = json.load(open(state / "deployed.json"))
-    assert reg["example-gpu-snapshot"]["path"] == SNAPSHOT
-    r = subprocess.run([sys.executable, SNAPSHOT], env=env, capture_output=True, text=True, timeout=300)
+    assert reg["example-gpu-snapshot"]["path"] == snapshot
+    r = subprocess.run([sys.executable, snapshot], env=env, capture_output=True, text=True, timeout=300)
     assert r.returncode == 0, (r.stdout[-2000:], r.stderr[-3000:])
     assert "calling Modal Function" in r.stdout and "loading model" in r.stdout and "snapshotting v1" in r.stdout
     vec = json.loads(r.stdout.strip().splitlines()[-1])
